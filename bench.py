@@ -10,6 +10,8 @@ the timed region.  L2 is flushed between timed steps (the 32 MB tableau is small
 a step the tableau legitimately stays L2-resident because every pivot rewrites all of it).
 
   python bench.py --gpus N --steps K --warmup W            # B200 arm
+  python bench.py ... --dump-outputs DIR                    # B200 arm, then the last timed step's outputs as
+        DIR/<name>.npy (final tableau, basis maps, status; e2e read-back; MIP solution), inputs fixed by --seed
   python bench.py --impl reference --gpus N --steps K ...   # CPU arm: the oracle restatement of the
         reference's TypeScript path (Node.js is not available), single thread, bounded sample.
 
@@ -37,9 +39,40 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the benchmark leaves the source tree as it found it (it may be read-only)
 
 METRIC = "pivots_per_sec_dense_lp_2000x2000_fp64"
 UNIT = "pivots/s"
+DUMP_BYTES = 64_000_000  # --dump-outputs budget over all files, .npy headers included
+
+
+def lp_status_array(st):
+    """What an LP solve reports besides the tableau, as float64 (the integers are exact)."""
+    import numpy as np
+    return np.array([st.feasible, st.bounded, st.evaluation, st.evaluation_raw, st.phase1_pivots, st.phase2_pivots],
+                    dtype=np.float64)
+
+
+def write_outputs(out_dir: str, arrays: dict) -> None:
+    """Writes each array as out_dir/<name>.npy in float64, DUMP_BYTES in all.  The budget is shared out smallest array
+    first; an array larger than its share is replaced by a fixed seeded sample of its elements (row-major flat order),
+    whose flat indices go to <name>_index.npy.  Same arguments, same files: two builds compare output for output."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    header = 128  # numpy writes a 128-byte header for these 1-D / 2-D float64 arrays
+    left, items = DUMP_BYTES, sorted(arrays.items(), key=lambda kv: np.asarray(kv[1]).size)
+    for i, (name, a) in enumerate(items):
+        a = np.asarray(a, dtype=np.float64)
+        share = left // (len(items) - i)
+        if a.nbytes + header <= share:
+            np.save(os.path.join(out_dir, f"{name}.npy"), a)
+            left -= a.nbytes + header
+            continue
+        n = (share - 2 * header) // 16  # value + index per sampled element
+        idx = np.sort(np.random.default_rng(0).choice(a.size, size=n, replace=False))
+        np.save(os.path.join(out_dir, f"{name}.npy"), a.reshape(-1)[idx])
+        np.save(os.path.join(out_dir, f"{name}_index.npy"), idx.astype(np.float64))
+        left -= 16 * n + 2 * header
 
 
 def algorithmic_bytes_per_pivot(H: int, W: int) -> int:
@@ -121,8 +154,10 @@ def l2_copy_peak(ctx, nbytes: int):
     return out.value
 
 
-def run_mip_leg(args, torch, dist, rank, world):
-    """BASELINE configs[4] through the public Model.solve(); returns the `mip` block (rank 0) or None."""
+def run_mip_leg(args, torch, dist, rank, world, outputs=None):
+    """BASELINE configs[4] through the public Model.solve(); returns the `mip` block (rank 0) or None.  With
+    `outputs`, the last repetition's solution is added to it."""
+    import numpy as np
     import jslpsolver_b200 as J
     from jslpsolver_b200 import problems
     model = problems.knapsack_mip_model(1024, 512, seed=12345)
@@ -162,6 +197,12 @@ def run_mip_leg(args, torch, dist, rank, world):
                "pivots_committed": b.pivots, "result": sol.evaluation, "collectives_per_rank": b.collectives,
                "nodes_pruned": b.nodes_pruned, "slot_pivots": int(slot_pivots), "slot_ms_max_rank": sl.item(),
                "slot_bytes": slot_bytes, "launches": int(launches)}
+        if outputs is not None and rep == args.mip_reps:  # read back before the tableau is closed
+            values = sol.generateSolutionSet()
+            outputs.update(mip_solution=np.array([values.get(v.id, 0.0) for v in inst.variables]),
+                           mip_rhs=inst.tableau.rhs_column(), mip_var_index_by_row=inst.tableau.varIndexByRow,
+                           mip_status=np.array([sol.feasible, sol.bounded, sol.evaluation, b.iterations, b.pivots],
+                                               dtype=np.float64))
         inst.tableau.close()
         if rep > 0 and (best is None or rec["total_ms"] < best["total_ms"]):
             best = rec
@@ -347,6 +388,10 @@ def run_b200(args, rank: int, world: int, local_rank: int):
     launches = ctx.launches - launches0
     clocks = sampler.stop()
     barrier()
+    outputs = {} if args.dump_outputs and rank == 0 else None
+    if outputs is not None:  # the last timed step's tableau, read back before the e2e arm overwrites it
+        outputs.update(lp_matrix=g.matrix2d(), lp_var_index_by_row=g.varIndexByRow,
+                       lp_var_index_by_col=g.varIndexByCol, lp_status=lp_status_array(last))
 
     # e2e: host buffers in, host buffers out, copies inside the timed region
     for _ in range(min(args.warmup, 2)):
@@ -363,12 +408,15 @@ def run_b200(args, rank: int, world: int, local_rank: int):
         e_ms += e0.elapsed_time(e1)
         e_pivots += st.phase1_pivots + st.phase2_pivots
     barrier()
+    if outputs is not None:
+        outputs.update(e2e_rhs=out_rhs.numpy().copy(), e2e_var_index_by_row=out_vr.numpy().copy(),
+                       e2e_var_index_by_col=out_vc.numpy().copy(), e2e_status=lp_status_array(st))
 
     l2_gbs = l2_copy_peak(ctx, H * W * 8) if rank == 0 else None
     mip = None
     if args.mip_nodes > 0:
         try:
-            mip = run_mip_leg(args, torch, dist, rank, world)
+            mip = run_mip_leg(args, torch, dist, rank, world, outputs)
         except Exception as e:  # the LP headline must not be lost to a failure of the secondary block
             if world > 1:
                 raise           # ... but a rank that drops out of the collectives must not leave the others waiting
@@ -422,6 +470,9 @@ def run_b200(args, rank: int, world: int, local_rank: int):
         }
         if mip is not None:
             line["mip"] = mip
+        if outputs is not None:
+            write_outputs(args.dump_outputs, outputs)
+            line["outputs"] = {"dir": args.dump_outputs, "arrays": sorted(outputs)}
         if world == 1 and not args.no_cpu:
             p, dt = cpu_sample(it, args.cpu_pivots)
             p2, dt2 = cpu_sample(it, args.cpu_pivots, check_cycles=False)
@@ -454,7 +505,14 @@ def main():
     ap.add_argument("--mip-nodes", type=int, default=1000, help="committed-node cap of the MIP block (0 = skip it)")
     ap.add_argument("--mip-spec", type=int, default=0, help="speculation width K (0 = 32 per GPU)")
     ap.add_argument("--mip-reps", type=int, default=2)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the timed paths returned in their last step to DIR/<name>.npy (float64, 64 MB "
+                         "at most) so that two builds can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs dumps the B200 arm's outputs")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

@@ -202,3 +202,25 @@ def test_napi_addon_compiles_against_the_header(tmp_path):
     methods = set(re.findall(r'\{"([A-Za-z0-9]+)", nullptr, tab_', cc))
     used = set(re.findall(r"this\.tab\(\)\.([A-Za-z0-9]+)\(", ts))
     assert used and used <= methods, used - methods
+
+
+def test_bench_output_dump_fits_its_budget_and_repeats(tmp_path, monkeypatch):
+    """bench.py --dump-outputs: small arrays are written whole as float64, an array beyond the 64 MB budget becomes a
+    fixed seeded sample of its elements with their flat indices, and the same arrays give the same files."""
+    import sys
+    monkeypatch.setattr(sys, "dont_write_bytecode", sys.dont_write_bytecode)  # bench.py sets it on import
+    import bench
+    big = np.arange(3001 * 3001, dtype=np.float64).reshape(3001, 3001)  # 72 MB: each value is its flat index
+    arrays = {"lp_matrix": big, "lp_var_index_by_row": np.arange(3001, dtype=np.int32), "lp_status": np.array([1, 1, -5.5])}
+    for d in ("a", "b"):
+        bench.write_outputs(str(tmp_path / d), arrays)
+    files = sorted(os.listdir(tmp_path / "a"))
+    assert files == ["lp_matrix.npy", "lp_matrix_index.npy", "lp_status.npy", "lp_var_index_by_row.npy"]
+    assert sum(os.path.getsize(tmp_path / "a" / f) for f in files) <= bench.DUMP_BYTES
+    for f in files:
+        assert (tmp_path / "a" / f).read_bytes() == (tmp_path / "b" / f).read_bytes(), f
+        assert np.load(tmp_path / "a" / f).dtype == np.float64, f
+    sample, idx = np.load(tmp_path / "a" / "lp_matrix.npy"), np.load(tmp_path / "a" / "lp_matrix_index.npy")
+    assert len(sample) > 3_000_000 and np.array_equal(sample, idx) and np.all(np.diff(idx) > 0)
+    assert np.array_equal(np.load(tmp_path / "a" / "lp_var_index_by_row.npy"), np.arange(3001))
+    assert np.array_equal(np.load(tmp_path / "a" / "lp_status.npy"), [1, 1, -5.5])
